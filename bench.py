@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the TEM-suite hot path (BASELINE.json metric: column.level.steps/s).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config config2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config config2] [--dump-outputs DIR]
 
 Headline (`value`, `ms_per_step`, `roofline`, `e2e`): one "step" = the full TEM suite (project -> fused
 eddy/flux/project -> output-grid synthesis -> stencil epilogue) over ONE 73-step time slab of config 2 with the four
@@ -21,6 +21,11 @@ Each carries its roofline fractions and a spot check of one time step against te
 
 `--impl reference` times the reference's CPU algorithm (the NumPy oracle port, factored form: the literal N x N operator
 of sph_zonal_mean.py:251 needs 956 GB at this grid) on a bounded sample.
+
+`--steps K` is the number of timed headline steps and of timed public-API calls in `e2e`.  `--dump-outputs DIR` writes
+what the last timed headline step computed (rank 0's slab) as DIR/<name>.npy, float64: every epilogue plane, on a fixed
+seeded sample of the slab's time steps that keeps the files within 64 MB.  The inputs are generated from a fixed seed,
+so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -45,6 +50,7 @@ FP64_PEAK_TFLOPS = 37.1   # measured DMMA m8n8k4 issue-rate peak on this pool (p
 PUBLIC = ('vtem', 'omegatem', 'wtem', 'psitem', 'epfy', 'epfz', 'epdiv', 'utendepfd', 'utendvtem', 'utendwtem')
 # (seed, time step) of the committed one-step expectations, tests/golden/make_scale_golden.py
 FIXTURES = {'config2': ('scale_config2_t1', 1, 182), 'config3': ('scale_config3_t1', 2, 48), 'config4': ('scale_config4_t1', 3, 120)}
+DUMP_BYTES = 64 * 10 ** 6       # cap on what --dump-outputs writes
 
 
 def peaks():
@@ -260,6 +266,24 @@ def spot_check(ctx, cfgname, res_planes, t_first, t_count):
             'max_normwise_err': err if err >= 0 else None, 'ok': bool(0 <= err < 1e-10)}
 
 
+def dump_outputs(path, res_planes, t_first):
+    """Writes res_planes (name -> [T_local][K][M] device tensors of the steps [t_first, t_first + T_local)) as
+    path/<name>.npy, float64, keeping a seeded sample of the time steps (the same one for every plane) so that the
+    files stay within DUMP_BYTES."""
+    import torch
+    first = next(iter(res_planes.values()))
+    step_bytes = sum(v[0].numel() * 8 for v in res_planes.values())
+    keep = min(first.shape[0], DUMP_BYTES // step_bytes)
+    assert keep >= 1, 'one time step of the outputs exceeds the --dump-outputs cap'
+    idx = np.sort(np.random.default_rng(0).choice(first.shape[0], keep, replace=False))
+    sel = torch.as_tensor(idx, device=first.device)
+    os.makedirs(path, exist_ok=True)
+    for n, v in res_planes.items():
+        np.save(os.path.join(path, n + '.npy'), v.index_select(0, sel).to(torch.float64).cpu().numpy())
+    return {'dir': path, 'arrays': sorted(res_planes), 'dtype': 'float64', 'time_steps': [t_first + int(i) for i in idx],
+            'shape': [keep] + list(first.shape[1:]), 'bytes': keep * step_bytes}
+
+
 def ev_pair(torch):
     return torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 
@@ -335,6 +359,7 @@ def headline(args, ctx):
     ms = ctx.max(e0.elapsed_time(e1) / args.steps)
     value = N * K * Ts * ctx.world / (ms * 1e-3)
     kms = {n: float(np.mean([a.elapsed_time(b) for a, b in v])) for n, v in ev.items()}
+    dump = dump_outputs(args.dump_outputs, res, t_off) if args.dump_outputs and ctx.rank == 0 else None
     check = spot_check(ctx, args.config, res, t_off, Ts) if fname else None
 
     Lp, rows = L + 1, Ts * K
@@ -358,7 +383,7 @@ def headline(args, ctx):
                  'achieved': fl_proj / (kms['project'] * 1e-3) / 1e12, 'peak': FP64_PEAK_TFLOPS, 'unit': 'TFLOP/s'}
     roof_proj['frac'] = roof_proj['achieved'] / roof_proj['peak']
     out = dict(cfg=cfg, L=L, N=N, K=K, Ts=Ts, ms=ms, value=value, kms=kms, clocks=clocks, basis_s=basis_s, roof=roof,
-               roof_proj=roof_proj, spot_check=check, launches_per_step=launches_per_step,
+               roof_proj=roof_proj, spot_check=check, launches_per_step=launches_per_step, dump=dump,
                step_tf=22.0 * Lp * N * rows / (ms * 1e-3) / 1e12,
                hbm={'bytes_per_point': 64, 'achieved_gbs': 64.0 * N * rows / (ms * 1e-3) / 1e9, 'peak_gbs': peaks().get('hbm_gbs')})
     return out, eng, xs, plev, lat
@@ -444,7 +469,7 @@ def e2e_leg(args, ctx, head, xs, plev, lat):
         for _ in range(2):
             call()
         ctx.barrier()
-        nrep = 5
+        nrep = args.steps
         a, b = ev_pair(torch)
         calls = []
         a.record()
@@ -747,6 +772,8 @@ def run_ours(args):
         'kernel_ms': head['kms'], 'basis_build_s': head['basis_s'], 'spot_check': head['spot_check'],
         'cpu_baseline': cpu, 'records': records,
     }
+    if head['dump']:
+        line['dump_outputs'] = head['dump']
     print(json.dumps(line))
     if ctx.world > 1:
         ctx.dist.destroy_process_group()
@@ -765,7 +792,13 @@ def main():
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-records', action='store_true', help='skip the config 3 / 4 / 5 record blocks')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed as DIR/<name>.npy (float64, at most 64 MB)')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
     if args.impl == 'reference':
         run_reference(args)
     else:

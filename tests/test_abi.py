@@ -3,7 +3,6 @@ import os
 import re
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -27,12 +26,18 @@ def test_epilogue_enum_matches_python():
 
 
 def test_no_gpu_means_loud_failure():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip('GPU present')
-    from pytemdiags_b200 import sph_zonal_averager
-    with pytest.raises(RuntimeError, match='no CPU fallback'):
-        sph_zonal_averager(np.linspace(-80, 80, 100), np.arange(-89.5, 90, 1.0), 10)
+    # in a child process that sees no CUDA device, so that this also runs on a machine with a GPU
+    import subprocess
+    import sys
+    code = '\n'.join([
+        'import sys; sys.path.insert(0, %r)' % ROOT,
+        'import numpy as np, pytest, torch',
+        'assert not torch.cuda.is_available()',
+        'from pytemdiags_b200 import sph_zonal_averager',
+        'with pytest.raises(RuntimeError, match="no CPU fallback"):',
+        '    sph_zonal_averager(np.linspace(-80, 80, 100), np.arange(-89.5, 90, 1.0), 10)',
+    ])
+    subprocess.check_call([sys.executable, '-c', code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=''))
 
 
 def test_product_never_imports_oracle():
