@@ -519,7 +519,7 @@ extern "C" int temd_synth_native(temd_plan* p, const double* coef, int rows, dou
     if (p == nullptr || !p->built) return temd_set_error(-1, "synth_native: basis not built");
     if (coef == nullptr || out == nullptr || rows < 1 || ld_out < (size_t)p->N) return temd_set_error(-1, "synth_native: bad arguments");
     TEMD_ON_DEVICE(p->dev);
-    static const bool use_res = [] { const char* e = getenv("TEMD_SYNTH_RESIDENT"); return !(e && atoi(e) == 0); }();
+    const bool use_res = [] { const char* e = getenv("TEMD_SYNTH_RESIDENT"); return !(e && atoi(e) == 0); }();   // read per call: A/B in one process
     if (use_res) {
         const int rc = launch_synth_resident(coef, rows, p->lpad, p->lpad, p->qt, p->N, p->ld_q, out, ld_out, p->sms,
                                              reinterpret_cast<cudaStream_t>(stream));
@@ -579,7 +579,7 @@ static int eddy_flux_impl(temd_plan* p, const double* const* x4, int rows, size_
     const bool can_fuse = eddy_supported(p->lpad) && (nprod == 3 || p->lpad <= 104);
     const bool split = (mode == 2) || !can_fuse || (mode == 0 && p->lpad > 104);
     if (!split) {
-        const int nsplit = eddy_pick_split(rows, p->lpad, nchunks, p->sms);
+        const int nsplit = eddy_pick_split(rows, p->lpad, nchunks, p->sms, nprod);
         double* work = nullptr;
         int rc = ensure_work(p, st, eddy_workspace_doubles(rows, p->lpad, nsplit, nprod), &work);
         if (rc) return rc;

@@ -352,7 +352,9 @@ k_eddy(const __grid_constant__ EddyMaps maps, const EddyParams p) {
 // warps of three different groups, and the smaller X tiles leave room for FIVE pipeline stages, i.e. 1.5 barrier rounds
 // of TMA look-ahead instead of one).  Measured on the config-2 slab: 80.4 ms against 78.5 ms for 8 fat warps - the
 // four-warps-per-group role split costs more shared-memory traffic than the extra look-ahead returns.
-static int eddy_bm(int nt) {
+// The tracer-pair kernel (nprod = 4) has only the BM = 32 layout: TEMD_EDDY_BM does not apply to it.
+static int eddy_bm(int nt, int nprod) {
+    if (nprod == 4) return 32;
     if (nt <= 13) {
         const char* e = getenv("TEMD_EDDY_BM");      // read per call: A/B in one process
         return (e && atoi(e) == 24) ? 24 : 32;
@@ -372,8 +374,8 @@ static int eddy_stages(int nt, int bm, int* smem_bytes) {
     return stages;
 }
 
-int eddy_pick_split(int rows, int lpad, int nchunks, int sms) {
-    const int bm = eddy_bm(lpad / 8);
+int eddy_pick_split(int rows, int lpad, int nchunks, int sms, int nprod) {
+    const int bm = eddy_bm(lpad / 8, nprod);
     return project_pick_split((rows + bm - 1) / bm, nchunks, sms, 64);
 }
 
@@ -407,7 +409,7 @@ int launch_eddy_flux_project(const double* const* x4, int rows, int ncol, size_t
     if (nprod != 3 && nprod != 4) return temd_set_error(-1, "eddy_flux_project: nprod must be 3 (TEM) or 4 (tracer pair)");
     if (!eddy_supported(lpad)) return temd_set_error(-1, "eddy_flux_project: L+1 > 408 is not supported by the fused kernel");
     const int nt = lpad / 8;
-    const int bm = eddy_bm(nt);
+    const int bm = eddy_bm(nt, nprod);
     EddyMaps maps;
     int rc;
     for (int f = 0; f < 4; f++)
@@ -440,7 +442,7 @@ int launch_eddy_flux_project(const double* const* x4, int rows, int ncol, size_t
     { const char* e = getenv("TEMD_EDDY_WARPS"); if (e && bm != 8 && bm != 24) warps = atoi(e) == 8 ? 8 : 16; }
     rc = -1;
     if (nprod == 4) {
-        if (bm != 32) return temd_set_error(-1, "eddy_flux_project: the tracer-pair kernel needs BM = 32 (L + 1 <= 104, TEMD_EDDY_BM unset)");
+        if (bm != 32) return temd_set_error(-1, "eddy_flux_project: the tracer-pair kernel needs BM = 32 (L + 1 <= 104)");
         p.nch = 1;
         const int nj = (nt + 1) / 2;
         switch (nj) {

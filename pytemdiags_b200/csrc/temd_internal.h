@@ -52,7 +52,7 @@ int launch_matmul_small(const double* A, const double* B, double* C, int n, int 
 
 // ---- K5 fused eddy / flux / projection (temd_eddy.cu) ----
 int eddy_supported(int lpad);
-int eddy_pick_split(int rows, int lpad, int nchunks, int sms);
+int eddy_pick_split(int rows, int lpad, int nchunks, int sms, int nprod);
 size_t eddy_workspace_doubles(int rows, int lpad, int nsplit, int nprod);
 int launch_eddy_flux_project(const double* const* x4, int rows, int ncol, size_t ld_x, const double* qt, int lpad,
                              size_t ld_q, const double* coef4, double* coef_flux, double* part, int nsplit,

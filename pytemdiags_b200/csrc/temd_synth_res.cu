@@ -166,8 +166,8 @@ int launch_synth_resident(const double* c, int rows, int lpad, size_t ld_c, cons
     const int nt = lpad / 8;
     // 64-row tiles (MTW = 1) with few enough stages that TWO CTAs share an SM: measured on the config-5 sweep
     // 0.845 vs 0.822 of the FP64 peak at L = 100, 0.725 vs 0.718 at L = 50, 0.599 vs 0.605 at L = 25
-    // (TEMD_SYNTH_RES_MTW=1|2 forces either).
-    static const int mtw_env = [] { const char* v = getenv("TEMD_SYNTH_RES_MTW"); return v ? atoi(v) : 0; }();
+    // (TEMD_SYNTH_RES_MTW=1|2 forces either; read per call, like TEMD_SYNTH_RES_NCH: A/B in one process).
+    const int mtw_env = [] { const char* v = getenv("TEMD_SYNTH_RES_MTW"); return v ? atoi(v) : 0; }();
     const int mtw = (mtw_env == 1 || (mtw_env != 2 && nt > 4)) ? 1 : 2;
     const int bm = SR_WARPS * 8 * mtw;
     SynthResParams p;
@@ -201,7 +201,7 @@ int launch_synth_resident(const double* c, int rows, int lpad, size_t ld_c, cons
         if (e != cudaSuccess) return temd_set_error((int)e, "synth_resident: cudaFuncSetAttribute failed");       \
         k_synth_res<M_, T_><<<ntiles * p.nsplit, SR_THREADS, smem, stream>>>(qmap, p);                             \
     } while (0)
-    static const int nch_env = [] { const char* v = getenv("TEMD_SYNTH_RES_NCH"); return v ? atoi(v) : 0; }();
+    const int nch_env = [] { const char* v = getenv("TEMD_SYNTH_RES_NCH"); return v ? atoi(v) : 0; }();
     int nch = (nt > 4) ? 2 : 1;
     if (nch_env == 1 || nch_env == 2 || nch_env == 4) nch = nch_env;
     if (nch == 4 && p.stages < 8) nch = 2;

@@ -44,8 +44,10 @@ def test_config1_full():
 
 @pytest.mark.parametrize('name', ['scale_config2_t1', 'scale_config3_t1', 'scale_config4_t1'])
 def test_big_config_one_step(name):
-    """configs 2 (ne120pg2, L=100), 3 (ne256pg2 x 128 lev, L=200: k_eddy BM=16) and 4 (721x1440 lat-lon, L=300:
-    k_eddy BM=8) at full column count, one time step of the record."""
+    """configs 2 (ne120pg2, L=100: fused k_eddy BM=32), 3 (ne256pg2 x 128 lev, L=200) and 4 (721x1440 lat-lon, L=300)
+    at full column count, one time step of the record.  Configs 3 and 4 have L + 1 > 104 and take the split eddy path
+    (k_synth eddy epilogue + product-mode k_project); the fused BM = 16 / 8 kernels are covered by
+    tests/test_gpu_instantiations.py."""
     from pytemdiags_b200 import TEMDiagnostics
     path = os.path.join(GOLD, name + '.npz')
     if not os.path.exists(path):
