@@ -35,6 +35,14 @@ int temd_plan_create(int device, int ncol, int L, int nlat_out, temd_plan** plan
 int temd_plan_destroy(temd_plan* plan);
 int temd_plan_lpad(const temd_plan* plan);
 
+/* Plan for temd_basis_build_min_norm: as temd_plan_create, but L+1 > ncol is allowed (a rank-deficient Y0 is then
+ * certain; the de-duplicated plan lives on U < L+1 unique nodes whenever the grid has fewer latitudes than degrees). */
+int temd_plan_create_min_norm(int device, int ncol, int L, int nlat_out, temd_plan** plan);
+
+/* Number of whitened basis directions of the built plan: L+1 after temd_basis_build / _dedup / _weighted, the rank r
+ * after temd_basis_build_min_norm; -1 if the basis is not built. */
+int temd_plan_rank(const temd_plan* plan);
+
 /* sph_zonal_averager.sph_compute_matrices (sph_zonal_mean.py:302-422): builds the Legendre basis at
  * x = cos(colatitude) of the native (x[N]) and output (x_out[M]) latitudes by three-term recurrence
  * (replaces sph_harm loops :359-370), the Gram matrix, its Cholesky factor, and the orthonormalised
@@ -42,6 +50,20 @@ int temd_plan_lpad(const temd_plan* plan);
  * sanity[0] = sum diag(Y0inv*Y0), sanity[1] = sum offdiag (the reference's logged check :393-398),
  * written to host memory if sanity_host != NULL. */
 int temd_basis_build(temd_plan* plan, const double* x, const double* x_out, double* sanity_host, void* stream);
+
+/* Minimum-norm least squares, for rank-deficient Y0 (e.g. more Legendre degrees than distinct latitudes): the result
+ * is NumPy's np.linalg.lstsq(Y0, ., rcond=None), i.e. Y0inv = pinv(Y0) with singular values sigma_i <=
+ * eps * max(N, L+1) * sigma_1 dropped (N = total column count, eps = 2^-52).  The rank decision comes from a one-sided
+ * Jacobi SVD of Yw = diag(sqrt(mult)) Y0(x_unique) (same singular values and right singular vectors as Y0); the basis
+ * is whitened with (V_r Sigma_r^-1)^T and re-orthonormalised by one Cholesky pass.  Coefficients r..lpad-1 are exactly
+ * zero, so every other entry point runs unchanged at the plan's lpad.
+ *   x        the plan's ncol nodes (dense plan), or NULL for a plan created on the unique nodes (the de-duplicated
+ *            path: its basis is then the weighted unique grid of temd_basis_build_dedup, and nunique = ncol);
+ *   x_unique, mult  the nunique distinct nodes and how many columns of the full grid share each (any order).
+ * rank_host (nullable): r.  sanity_host as in temd_basis_build, with sanity[0] = r.  Fails (<0) if the Jacobi sweeps
+ * do not converge or the rank-r whitened basis is not positive definite.  Works on any plan. */
+int temd_basis_build_min_norm(temd_plan* plan, const double* x, const double* x_unique, const double* mult, int nunique,
+                              const double* x_out, int* rank_host, double* sanity_host, void* stream);
 
 /* Deprecated quadrature inverse of the reference, Y0inv = Y0^T diag(w) (sph_zonal_mean.py:72,180-181,383-386):
  * w[N] are the grid-cell area weights ALREADY multiplied by 4 pi.  temd_project / temd_synth_* then compute

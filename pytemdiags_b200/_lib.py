@@ -16,6 +16,7 @@ SYMBOLS = (
     'temd_eddy_native', 'temd_multiply', 'temd_eddy_flux_project', 'temd_tracer_flux_project', 'temd_tem_epilogue', 'temd_tracer_epilogue', 'temd_check_finite', 'temd_host_copy', 'temd_synth_fields',
     'temd_synth_out_dlat', 'temd_basis_export_dlat', 'temd_basis_build_dedup', 'temd_group_sums', 'temd_dedup_flux', 'temd_dedup_expand',
     'temd_comm_unique_id', 'temd_comm_init', 'temd_comm_destroy', 'temd_allgather_outputs',
+    'temd_plan_create_min_norm', 'temd_plan_rank', 'temd_basis_build_min_norm',
 )
 
 # order of the output planes written by temd_tem_epilogue (enum TEMD_OUT_* in temd.h)
@@ -86,6 +87,9 @@ def load():
     lib.temd_plan_create.argtypes = [i, i, i, i, C.POINTER(vp)]
     lib.temd_plan_destroy.argtypes = [vp]
     lib.temd_plan_lpad.argtypes = [vp]
+    lib.temd_plan_create_min_norm.argtypes = [i, i, i, i, C.POINTER(vp)]
+    lib.temd_plan_rank.argtypes = [vp]
+    lib.temd_basis_build_min_norm.argtypes = [vp, vp, vp, vp, i, vp, C.POINTER(i), C.POINTER(d), vp]
     lib.temd_basis_build.argtypes = [vp, vp, vp, C.POINTER(d), vp]
     lib.temd_basis_build_weighted.argtypes = [vp, vp, vp, vp, vp]
     lib.temd_basis_export.argtypes = [vp, vp, vp, vp, vp]

@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libtemd.so')
 SOURCES = ['temd_api.cu', 'temd_project.cu', 'temd_basis.cu', 'temd_synth.cu', 'temd_synth_res.cu', 'temd_eddy.cu',
-           'temd_epilogue.cu', 'temd_fields.cu', 'temd_comm.cu', 'temd_dedup.cu']
+           'temd_epilogue.cu', 'temd_fields.cu', 'temd_comm.cu', 'temd_dedup.cu', 'temd_svd.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr']
 

@@ -194,6 +194,7 @@ struct temd_plan {
     double* sanity;
     bool built;
     bool weighted;   // deprecated quadrature inverse Y0inv = Y0^T diag(w): qt = raw basis (synthesis), qt_alt = weighted (projection)
+    int rank;        // number of whitened directions of the built basis (L+1 unless built by temd_basis_build_min_norm)
 };
 
 // Split-K workspace of `stream` (grown on demand).  Work already enqueued on that stream may still use the old
@@ -217,12 +218,12 @@ static size_t round_up(size_t v, size_t m) { return (v + m - 1) / m * m; }
 extern "C" int temd_version(void) { return 101; }
 extern "C" const char* temd_last_error(void) { return g_err; }
 
-extern "C" int temd_plan_create(int device, int ncol, int L, int nlat_out, temd_plan** out) {
+static int plan_create_impl(int device, int ncol, int L, int nlat_out, bool min_norm, temd_plan** out) {
     if (out == nullptr) return temd_set_error(-1, "plan_create: null output");
     *out = nullptr;
     if (ncol < 1 || L < 0 || nlat_out < 1) return temd_set_error(-1, "plan_create: bad sizes (ncol %d, L %d, M %d)", ncol, L, nlat_out);
     if (L + 1 > 1024) return temd_set_error(-1, "plan_create: L = %d exceeds the supported maximum 1023", L);
-    if (L + 1 > ncol) return temd_set_error(-1, "plan_create: L+1 = %d exceeds ncol = %d (Y0 would be rank-deficient: lower L; the reference's lstsq would return a minimum-norm solution here, this build does not)", L + 1, ncol);
+    if (!min_norm && L + 1 > ncol) return temd_set_error(-1, "plan_create: L+1 = %d exceeds ncol = %d (Y0 would be rank-deficient: lower L; the reference's lstsq would return a minimum-norm solution here, this build does not)", L + 1, ncol);
     TEMD_ON_DEVICE(device);
     cudaDeviceProp prop;
     TEMD_CUDA(cudaGetDeviceProperties(&prop, device));
@@ -232,6 +233,7 @@ extern "C" int temd_plan_create(int device, int ncol, int L, int nlat_out, temd_
     p->work_mu = new std::mutex();
     p->work = new std::map<std::pair<cudaStream_t, int>, std::pair<double*, size_t>>();
     p->dev = device; p->N = ncol; p->L = L; p->Lp = L + 1; p->M = nlat_out;
+    p->rank = -1;
     p->lpad = (int)round_up(L + 1, 8);
     p->sms = prop.multiProcessorCount;
     p->ld_q = round_up(ncol, 16);
@@ -254,6 +256,14 @@ extern "C" int temd_plan_create(int device, int ncol, int L, int nlat_out, temd_
     return 0;
 }
 
+extern "C" int temd_plan_create(int device, int ncol, int L, int nlat_out, temd_plan** out) {
+    return plan_create_impl(device, ncol, L, nlat_out, false, out);
+}
+
+extern "C" int temd_plan_create_min_norm(int device, int ncol, int L, int nlat_out, temd_plan** out) {
+    return plan_create_impl(device, ncol, L, nlat_out, true, out);
+}
+
 extern "C" int temd_plan_destroy(temd_plan* p) {
     if (p == nullptr) return 0;
     DeviceGuard guard(p->dev);
@@ -269,6 +279,7 @@ extern "C" int temd_plan_destroy(temd_plan* p) {
 }
 
 extern "C" int temd_plan_lpad(const temd_plan* p) { return p ? p->lpad : -1; }
+extern "C" int temd_plan_rank(const temd_plan* p) { return (p && p->built) ? p->rank : -1; }
 
 static int gram_of(temd_plan* p, const double* basis, cudaStream_t st) {
     int ntb, lblocks;
@@ -283,14 +294,9 @@ static int gram_of(temd_plan* p, const double* basis, cudaStream_t st) {
     return launch_project(xs, 1, p->Lp, p->N, p->ld_q, basis, p->lpad, p->ld_q, p->gram, work, nsplit, nullptr, -1, 1, st);
 }
 
-// `mult` (nullable): multiplicity of every node.  The raw basis rows are then scaled by sqrt(mult) before the
-// factorisation (weighted unique grid of the de-duplicated fast path, temd_dedup.cu): its Gram matrix is the Gram
-// matrix of the full grid in which node u appears mult[u] times.
-static int basis_build_impl(temd_plan* p, const double* x, const double* x_out, const double* mult, double* sanity_host,
-                            void* stream) {
-    if (p == nullptr || x == nullptr || x_out == nullptr) return temd_set_error(-1, "basis_build: null argument");
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    TEMD_ON_DEVICE(p->dev);
+// Recurrence coefficients, copies of the nodes and the raw (transposed) basis on both grids in qt_alt / qpt_alt;
+// `mult` (nullable) scales the native rows by sqrt(mult).  Runs on the caller's device and stream.
+static int raw_basis(temd_plan* p, const double* x, const double* x_out, const double* mult, cudaStream_t st) {
     // recurrence coefficients: Y_l = a_l x Y_{l-1} - b_l Y_{l-2}
     std::vector<double> ra(p->lpad, 0.0), rb(p->lpad, 0.0);
     const double PI = 3.141592653589793238462643383279502884;
@@ -314,6 +320,37 @@ static int basis_build_impl(temd_plan* p, const double* x, const double* x_out, 
         k_scale_cols_sqrt<<<grid, 256, 0, st>>>(p->qt_alt, mult, p->lpad, p->N, p->ld_q);
         TEMD_CUDA(cudaGetLastError());
     }
+    return 0;
+}
+
+// Optional sanity readback, then marks the whitened basis built with `rank` directions.
+static int finish_build(temd_plan* p, double* sanity_host, int rank, cudaStream_t st) {
+    int rc;
+    if (sanity_host != nullptr) {
+        // reference's logged check (sph_zonal_mean.py:393-398): Y0inv Y0 = L^-T (Q^T Q) L^T; we report Q^T Q
+        if ((rc = gram_of(p, p->qt, st))) return rc;
+        k_trace_offdiag<<<1, 256, 0, st>>>(p->gram, p->Lp, p->lpad, p->sanity);
+        TEMD_CUDA(cudaGetLastError());
+        TEMD_CUDA(cudaMemcpyAsync(sanity_host, p->sanity, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    }
+    TEMD_CUDA(cudaStreamSynchronize(st));
+    p->built = true;
+    p->weighted = false;
+    p->dqpt_built = false;
+    p->rank = rank;
+    return 0;
+}
+
+// `mult` (nullable): multiplicity of every node.  The raw basis rows are then scaled by sqrt(mult) before the
+// factorisation (weighted unique grid of the de-duplicated fast path, temd_dedup.cu): its Gram matrix is the Gram
+// matrix of the full grid in which node u appears mult[u] times.
+static int basis_build_impl(temd_plan* p, const double* x, const double* x_out, const double* mult, double* sanity_host,
+                            void* stream) {
+    if (p == nullptr || x == nullptr || x_out == nullptr) return temd_set_error(-1, "basis_build: null argument");
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    TEMD_ON_DEVICE(p->dev);
+    int rc = raw_basis(p, x, x_out, mult, st);
+    if (rc) return rc;
     // CholeskyQR2: G = Y^T Y = L L^T, Y <- Y L^-T, twice (the second pass removes the cond(Y0)^2 eps loss of
     // orthogonality of the first); L^-1 accumulates as L2^-1 L1^-1.  If the first factorisation breaks down
     // (cond(Y0) >~ 3e6), a shifted first pass (G + s I, s = 11 (N Lp + Lp(Lp+1)) eps trace(G), "shifted
@@ -357,17 +394,7 @@ static int basis_build_impl(temd_plan* p, const double* x, const double* x_out, 
             std::swap(p->linv, p->linv1);
         }
     }
-    if (sanity_host != nullptr) {
-        // reference's logged check (sph_zonal_mean.py:393-398): Y0inv Y0 = L^-T (Q^T Q) L^T; we report Q^T Q
-        if ((rc = gram_of(p, p->qt, st))) return rc;
-        k_trace_offdiag<<<1, 256, 0, st>>>(p->gram, p->Lp, p->lpad, p->sanity);
-        TEMD_CUDA(cudaGetLastError());
-        TEMD_CUDA(cudaMemcpyAsync(sanity_host, p->sanity, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    }
-    TEMD_CUDA(cudaStreamSynchronize(st));
-    p->built = true;
-    p->weighted = false;
-    p->dqpt_built = false;
+    if ((rc = finish_build(p, sanity_host, p->Lp, st))) return rc;
     return 0;
 }
 
@@ -379,6 +406,86 @@ extern "C" int temd_basis_build_dedup(temd_plan* p, const double* x_unique, cons
                                       double* sanity_host, void* stream) {
     if (mult == nullptr) return temd_set_error(-1, "basis_build_dedup: null multiplicities");
     return basis_build_impl(p, x_unique, x_out, mult, sanity_host, stream);
+}
+
+// Minimum-norm build: the first whitening pass uses W^T = (V_r Sigma_r^-1)^T from the Jacobi SVD of the weighted
+// unique-node basis Yw (temd_svd.cu) instead of L^-1; rows r..lpad-1 of every whitened basis are zero.  One Cholesky
+// pass on the leading r x r block then removes the cond_r eps loss of orthogonality of the first.
+extern "C" int temd_basis_build_min_norm(temd_plan* p, const double* x, const double* x_unique, const double* mult,
+                                         int nunique, const double* x_out, int* rank_host, double* sanity_host,
+                                         void* stream) {
+    if (p == nullptr || x_unique == nullptr || mult == nullptr || x_out == nullptr || nunique < 1)
+        return temd_set_error(-1, "basis_build_min_norm: null argument or nunique < 1");
+    if (x == nullptr && nunique != p->N)
+        return temd_set_error(-1, "basis_build_min_norm: x = NULL (plan on the unique nodes) needs nunique = ncol = %d, got %d",
+                              p->N, nunique);
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    TEMD_ON_DEVICE(p->dev);
+    p->built = false;
+    int rc = raw_basis(p, x ? x : x_unique, x_out, x ? nullptr : mult, st);
+    if (rc) return rc;
+    // Yw^T [lpad][ld_u] on the unique nodes; the vectors the SVD rotates are its rows (tall) or its columns (wide)
+    const int U = nunique, Lp = p->Lp, lpad = p->lpad;
+    const bool tall = U >= Lp;
+    const size_t ld_u = round_up(U, 16);
+    struct Scratch {
+        void* ptr = nullptr;
+        ~Scratch() { if (ptr) cudaFree(ptr); }
+    } scratch;
+    const size_t ywt_d = (size_t)lpad * ld_u, a_d = tall ? 0 : (size_t)U * lpad, vt_d = tall ? (size_t)lpad * lpad : 0;
+    const size_t total_d = ywt_d + a_d + vt_d + 2 * (size_t)lpad;
+    TEMD_CUDA(cudaMalloc(&scratch.ptr, total_d * sizeof(double) + 2 * sizeof(unsigned long long)));
+    double* ywt = static_cast<double*>(scratch.ptr);
+    double* a = ywt + ywt_d;
+    double* vt = a + a_d;
+    double* sigma = vt + vt_d;
+    double* sigma_sorted = sigma + lpad;
+    unsigned long long* off = reinterpret_cast<unsigned long long*>(sigma_sorted + lpad);
+    if ((rc = launch_basis(x_unique, U, p->L, p->rec_a, p->rec_b, ywt, ld_u, lpad, st))) return temd_set_error(rc, "basis kernel launch failed");
+    {
+        dim3 grid((unsigned)((ld_u + 255) / 256), lpad);
+        k_scale_cols_sqrt<<<grid, 256, 0, st>>>(ywt, mult, lpad, U, ld_u);
+        TEMD_CUDA(cudaGetLastError());
+    }
+    int sweeps = 0;
+    if (tall) {
+        if ((rc = launch_identity(vt, lpad, lpad, st))) return temd_set_error(rc, "identity launch failed");
+        rc = jacobi_svd_whitening(ywt, ld_u, U, Lp, vt, lpad, Lp, mult, U, p->linv2, lpad, sigma, sigma_sorted, p->status,
+                                  off, &sweeps, st);
+    } else {
+        dim3 tb(32, 8), grid((U + 31) / 32, (Lp + 31) / 32);
+        k_transpose<<<grid, tb, 0, st>>>(ywt, Lp, U, ld_u, a, lpad);
+        TEMD_CUDA(cudaGetLastError());
+        rc = jacobi_svd_whitening(a, lpad, Lp, U, nullptr, 0, Lp, mult, U, p->linv2, lpad, sigma, sigma_sorted, p->status,
+                                  off, &sweeps, st);
+    }
+    if (rc) return rc;
+    int rank = 0;
+    TEMD_CUDA(cudaMemcpyAsync(&rank, p->status, sizeof(int), cudaMemcpyDeviceToHost, st));
+    TEMD_CUDA(cudaStreamSynchronize(st));
+    if (rank < 1 || rank > Lp) return temd_set_error(-5, "basis_build_min_norm: rank %d outside [1, %d]", rank, Lp);
+    // pass 1: Q^T = W^T Y^T on both grids, written to qt / qpt
+    if ((rc = launch_synth(p->linv2, lpad, lpad, lpad, p->qt_alt, p->N, p->ld_q, p->qt, p->ld_q, st))) return rc;
+    if ((rc = launch_synth(p->linv2, lpad, lpad, lpad, p->qpt_alt, p->M, p->ld_p, p->qpt, p->ld_p, st))) return rc;
+    TEMD_CUDA(cudaMemcpyAsync(p->linv, p->linv2, (size_t)lpad * lpad * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    // pass 2: Cholesky of the leading r x r block of Q^T Q
+    if ((rc = gram_of(p, p->qt, st))) return rc;
+    if ((rc = launch_chol_inv(p->gram, lpad, rank, p->lt, p->linv2, lpad, lpad, p->status, st))) return temd_set_error(rc, "cholesky launch failed");
+    int status = 0;
+    TEMD_CUDA(cudaMemcpyAsync(&status, p->status, sizeof(int), cudaMemcpyDeviceToHost, st));
+    TEMD_CUDA(cudaStreamSynchronize(st));
+    if (status != 0)
+        return temd_set_error(-5, "basis_build_min_norm: Cholesky pivot %d of the rank-%d whitened basis non-positive "
+                                  "(L = %d)", status - 1, rank, p->L);
+    if ((rc = launch_synth(p->linv2, lpad, lpad, lpad, p->qt, p->N, p->ld_q, p->qt_alt, p->ld_q, st))) return rc;
+    if ((rc = launch_synth(p->linv2, lpad, lpad, lpad, p->qpt, p->M, p->ld_p, p->qpt_alt, p->ld_p, st))) return rc;
+    std::swap(p->qt, p->qt_alt);
+    std::swap(p->qpt, p->qpt_alt);
+    if ((rc = launch_matmul_small(p->linv2, p->linv, p->linv1, lpad, lpad, st))) return temd_set_error(rc, "matmul launch failed");
+    std::swap(p->linv, p->linv1);
+    if ((rc = finish_build(p, sanity_host, rank, st))) return rc;
+    if (rank_host != nullptr) *rank_host = rank;
+    return 0;
 }
 
 extern "C" int temd_basis_build_weighted(temd_plan* p, const double* x, const double* x_out, const double* w, void* stream) {
@@ -408,6 +515,7 @@ extern "C" int temd_basis_build_weighted(temd_plan* p, const double* x, const do
     p->built = true;
     p->weighted = true;
     p->dqpt_built = false;
+    p->rank = p->Lp;
     return 0;
 }
 

@@ -50,6 +50,16 @@ int launch_chol_inv(const double* G, int ldg, int n, double* LT, double* Linv, i
                     cudaStream_t stream);
 int launch_matmul_small(const double* A, const double* B, double* C, int n, int ld, cudaStream_t stream);
 
+// ---- one-sided Jacobi SVD for the minimum-norm build (temd_svd.cu) ----
+int launch_identity(double* M, int n, int ld, cudaStream_t stream);
+// Orthogonalises the k rows (length m) of A in place (Vt != NULL: accumulates the rotations into the k x k rows of Vt,
+// which must hold the identity), then writes the truncated whitening matrix Wt [lpad][lpad] and the rank (device
+// int).  sigma / sigma_sorted: k doubles each.  mult[nu]: node multiplicities (their sum is N in the cutoff).
+// Synchronises once per sweep; fails if the sweeps do not converge.
+int jacobi_svd_whitening(double* A, size_t lda, int m, int k, double* Vt, size_t ldv, int Lp, const double* mult,
+                         int nu, double* Wt, int lpad, double* sigma, double* sigma_sorted, int* rank_dev,
+                         unsigned long long* off_dev, int* sweeps_out, cudaStream_t stream);
+
 // ---- K5 fused eddy / flux / projection (temd_eddy.cu) ----
 int eddy_supported(int lpad);
 int eddy_pick_split(int rows, int lpad, int nchunks, int sms, int nprod);

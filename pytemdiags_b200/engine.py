@@ -48,10 +48,21 @@ def _check_rank(lat, L):
                                L + 1, np.unique(lat).shape[0], lat.shape[0], np.unique(lat).shape[0] - 1))
 
 
-class Engine:
-    """One zonal-averaging plan (native grid, output grid, truncation L) on one GPU."""
+def _unique_nodes(lat):
+    """x = cos(colatitude) of every column, computed like the reference (sph_zonal_mean.py:358), and its distinct
+    values: (x, x_unique, inverse, counts) as np.unique returns them."""
+    x = np.cos(np.deg2rad(90 - lat))
+    xu, inv, cnt = np.unique(x, return_inverse=True, return_counts=True)
+    return x, xu, inv, cnt
 
-    def __init__(self, lat, lat_out, L, device=None):
+
+class Engine:
+    """One zonal-averaging plan (native grid, output grid, truncation L) on one GPU.
+
+    `min_norm=True`: the basis is built by temd_basis_build_min_norm, so a rank-deficient Y0 gives NumPy's
+    minimum-norm least-squares answer instead of an error; `rank` is then the number of directions kept."""
+
+    def __init__(self, lat, lat_out, L, device=None, min_norm=False):
         self.lib = _lib.load()
         if not torch.cuda.is_available():
             raise RuntimeError('pytemdiags_b200 needs a CUDA device (sm_100a); there is no CPU fallback')
@@ -60,14 +71,36 @@ class Engine:
         self.lat_out = np.ascontiguousarray(np.asarray(lat_out, dtype=np.float64))
         self.N, self.M, self.L = int(self.lat.shape[0]), int(self.lat_out.shape[0]), int(L)
         self.Mld = self.M + (self.M & 1)
-        _check_rank(self.lat, self.L)
+        self.min_norm = bool(min_norm)
+        if not self.min_norm:
+            _check_rank(self.lat, self.L)
         self._plan = C.c_void_p(0)
-        _lib.check(self.lib.temd_plan_create(self.device.index or 0, self.N, self.L, self.M, C.byref(self._plan)),
-                   'temd_plan_create')
-        self.lpad = self.lib.temd_plan_lpad(self._plan)
+        self._create_plan(self.N)
         self.built = False
         self.sanity = None
+        self.rank = None
         self.lock = threading.RLock()   # serialises callers that share this (cached) engine's per-call state
+
+    def _create_plan(self, ncol):
+        create = self.lib.temd_plan_create_min_norm if self.min_norm else self.lib.temd_plan_create
+        _lib.check(create(self.device.index or 0, ncol, self.L, self.M, C.byref(self._plan)),
+                   'temd_plan_create_min_norm' if self.min_norm else 'temd_plan_create')
+        self.lpad = self.lib.temd_plan_lpad(self._plan)
+
+    def _build_min_norm(self, x, xu, cnt, x_out, sanity):
+        """temd_basis_build_min_norm; x = None on a plan created on the unique nodes."""
+        xu_d, mult = self._dev(xu), self._dev(cnt.astype(np.float64))
+        san = (C.c_double * 2)()
+        rank = C.c_int(0)
+        with torch.cuda.device(self.device):
+            rc = self.lib.temd_basis_build_min_norm(self._plan, _ptr(x), _ptr(xu_d), _ptr(mult), int(xu.shape[0]),
+                                                    _ptr(x_out), C.byref(rank), san if sanity else None, self.stream)
+        _lib.check(rc, 'temd_basis_build_min_norm')
+        self.built = True
+        self.rank = int(rank.value)
+        if sanity:
+            self.sanity = (san[0], san[1])
+        return self
 
     def __del__(self):
         try:
@@ -86,9 +119,14 @@ class Engine:
 
     # ---- sph_compute_matrices (sph_zonal_mean.py:302-422) ----
     def build_basis(self, sanity=False, weights=None):
+        if self.min_norm and weights is not None:
+            raise RuntimeError('min_norm=True is not available together with weights=')
         # x = cos(colatitude), computed exactly like the reference: coalt = deg2rad(90 - lat)
         x = self._dev(np.cos(np.deg2rad(90 - self.lat)))
         x_out = self._dev(np.cos(np.deg2rad(90 - self.lat_out)))
+        if self.min_norm:
+            _, xu, _, cnt = _unique_nodes(self.lat)
+            return self._build_min_norm(x, xu, cnt, x_out, sanity)
         if weights is not None:
             # deprecated reference path: Y0inv = Y0^T diag(4 pi w)  (sph_zonal_mean.py:180-181,383-386)
             w = self._dev(4 * np.pi * np.asarray(weights, dtype=np.float64))
@@ -96,12 +134,14 @@ class Engine:
                 rc = self.lib.temd_basis_build_weighted(self._plan, _ptr(x), _ptr(x_out), _ptr(w), self.stream)
             _lib.check(rc, 'temd_basis_build_weighted')
             self.built = True
+            self.rank = self.L + 1
             return self
         san = (C.c_double * 2)()
         with torch.cuda.device(self.device):
             rc = self.lib.temd_basis_build(self._plan, _ptr(x), _ptr(x_out), san if sanity else None, self.stream)
         _lib.check(rc, 'temd_basis_build')
         self.built = True
+        self.rank = self.L + 1
         if sanity:
             self.sanity = (san[0], san[1])
         return self
@@ -354,7 +394,7 @@ class DedupEngine(Engine):
     x = sin(lat); fields are reduced to per-group sums in ONE pass (csrc/temd_dedup.cu) and every tensor-core kernel
     runs on U columns instead of N.  Same method surface and the same coefficients (to rounding) as `Engine`."""
 
-    def __init__(self, lat, lat_out, L, device=None):
+    def __init__(self, lat, lat_out, L, device=None, min_norm=False):
         self.lib = _lib.load()
         if not torch.cuda.is_available():
             raise RuntimeError('pytemdiags_b200 needs a CUDA device (sm_100a); there is no CPU fallback')
@@ -363,11 +403,11 @@ class DedupEngine(Engine):
         self.lat_out = np.ascontiguousarray(np.asarray(lat_out, dtype=np.float64))
         self.N, self.M, self.L = int(self.lat.shape[0]), int(self.lat_out.shape[0]), int(L)
         self.Mld = self.M + (self.M & 1)
+        self.min_norm = bool(min_norm)
         # group the columns by the exact value of the basis argument (computed like the reference: sph_zonal_mean.py:358)
-        x = np.cos(np.deg2rad(90 - self.lat))
-        xu, inv, cnt = np.unique(x, return_inverse=True, return_counts=True)
+        x, xu, inv, cnt = _unique_nodes(self.lat)
         self.NU = int(xu.shape[0])
-        if self.NU < self.L + 1:
+        if self.NU < self.L + 1 and not self.min_norm:
             _check_rank(self.lat, self.L)
         self.Uld = self.NU + (self.NU & 1)
         self.multiplicity = self.N / self.NU
@@ -392,25 +432,28 @@ class DedupEngine(Engine):
         self._goff, self._gid = i32(goff), i32(inv)
         self._mult = self._dev(cnt.astype(np.float64))
         self._rsq = self._dev(1.0 / np.sqrt(cnt.astype(np.float64)))
+        self._cnt = cnt
         self._plan = C.c_void_p(0)
-        _lib.check(self.lib.temd_plan_create(self.device.index or 0, self.NU, self.L, self.M, C.byref(self._plan)),
-                   'temd_plan_create')
-        self.lpad = self.lib.temd_plan_lpad(self._plan)
+        self._create_plan(self.NU)
         self.built = False
         self.sanity = None
+        self.rank = None
         self.lock = threading.RLock()
 
     def build_basis(self, sanity=False, weights=None):
         if weights is not None:
             raise RuntimeError('dedup=True is not available with the deprecated quadrature-weights inverse')
-        xu = self._dev(self._xu)
         x_out = self._dev(np.cos(np.deg2rad(90 - self.lat_out)))
+        if self.min_norm:
+            return self._build_min_norm(None, self._xu, self._cnt, x_out, sanity)
+        xu = self._dev(self._xu)
         san = (C.c_double * 2)()
         with torch.cuda.device(self.device):
             rc = self.lib.temd_basis_build_dedup(self._plan, _ptr(xu), _ptr(x_out), _ptr(self._mult),
                                                  san if sanity else None, self.stream)
         _lib.check(rc, 'temd_basis_build_dedup')
         self.built = True
+        self.rank = self.L + 1
         if sanity:
             self.sanity = (san[0], san[1])
         return self

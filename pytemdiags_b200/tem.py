@@ -79,11 +79,13 @@ class TEMDiagnostics:
         p : 1-D pressure levels (hPa unless p_units='Pa') or a gridpoint pressure field in Pa that is
             constant on each level (pressure-level data).  Mandatory for raw arrays.
         Extra keywords of this build: dims, p, p_units, time, device, slab_bytes, dedup (structure-exploiting fast
-        path for grids with repeated latitudes, see sph_zonal_averager; default False).
+        path for grids with repeated latitudes, see sph_zonal_averager; default False), min_norm (minimum-norm
+        least squares on a rank-deficient basis, see sph_zonal_averager; default False; `rank` then tells how many
+        directions were kept).
         '''
         opts = dict(_DEFAULTS)
-        extra = {k: kwargs.pop(k) for k in ('dims', 'p', 'p_units', 'time', 'device', 'slab_bytes', 'lat', 'dedup')
-                 if k in kwargs}
+        extra = {k: kwargs.pop(k) for k in ('dims', 'p', 'p_units', 'time', 'device', 'slab_bytes', 'lat', 'dedup',
+                                            'min_norm') if k in kwargs}
         pos = list(args)
         ncol_guess = None
         # README shape: (p, lat, ...) -- the 6th positional is a 1-D latitude vector
@@ -131,6 +133,7 @@ class TEMDiagnostics:
         self._device = extra.get('device')
         self._slab_bytes = extra.get('slab_bytes')
         self._dedup = bool(extra.get('dedup', False))
+        self._min_norm = bool(extra.get('min_norm', False))
 
         self._config_dims()
 
@@ -138,12 +141,18 @@ class TEMDiagnostics:
         self.ZM = sph_zonal_averager(self._lat_native_np, self._lat_zm, self.L, grid_name=self.grid_name,
                                      grid_out_name=self.zm_grid_name, save_dest=self.map_save_dest,
                                      debug=self.debug_level > 1, overwrite=self.overwrite_map,
-                                     ncoldim=self.ncolname, device=self._device, dedup=self._dedup)
+                                     ncoldim=self.ncolname, device=self._device, dedup=self._dedup,
+                                     min_norm=self._min_norm)
         self.ZM.sph_compute_matrices(overwrite=self.overwrite_map)
         self._zonal_mean = self.ZM.sph_zonal_mean
 
         self._compute_all()
         self._out_file = None
+
+    @property
+    def rank(self):
+        '''Number of basis directions of the zonal averager: L+1, or the numerical rank of Y0 with min_norm=True.'''
+        return self.ZM.rank
 
     # ------------------------------------------------------------------
     def _log(self, s):

@@ -18,19 +18,19 @@ _ENGINE_CACHE = {}
 _ENGINE_CACHE_MAX = int(os.environ.get('TEMD_ENGINE_CACHE', '4'))   # plans kept (2.6 GB of basis each at config 3)
 
 
-def _cached_engine(lat, lat_out, L, device, overwrite=False, weights=None, dedup=False):
+def _cached_engine(lat, lat_out, L, device, overwrite=False, weights=None, dedup=False, min_norm=False):
     import hashlib
     dev = torch.device('cuda', torch.cuda.current_device()) if device is None else torch.device(device)
     wkey = None if weights is None else hashlib.sha1(np.ascontiguousarray(weights, dtype=np.float64).tobytes()).hexdigest()
     key = (hashlib.sha1(lat.tobytes()).hexdigest(), hashlib.sha1(lat_out.tobytes()).hexdigest(), int(L), str(dev), wkey,
-           bool(dedup))
+           bool(dedup), bool(min_norm))
     if overwrite:
         _ENGINE_CACHE.pop(key, None)
     eng = _ENGINE_CACHE.get(key)
     if eng is None:
         while len(_ENGINE_CACHE) >= _ENGINE_CACHE_MAX:
             _ENGINE_CACHE.pop(next(iter(_ENGINE_CACHE)))
-        eng = (DedupEngine if dedup else Engine)(lat, lat_out, L, device=dev)
+        eng = (DedupEngine if dedup else Engine)(lat, lat_out, L, device=dev, min_norm=min_norm)
         _ENGINE_CACHE[key] = eng
     return eng
 
@@ -41,7 +41,8 @@ DEFAULT_LAT_ATTRS = {'long_name': 'Latitude of Grid Cell Centers', 'standard_nam
 
 class sph_zonal_averager:
     def __init__(self, lat, lat_out, L, weights=None, grid_name=None, grid_out_name=None,
-                 ncoldim='ncol', overwrite=False, save_dest=None, debug=False, logfile=None, device=None, dedup=False):
+                 ncoldim='ncol', overwrite=False, save_dest=None, debug=False, logfile=None, device=None, dedup=False,
+                 min_norm=False):
         '''
         Zonal averages of fields on unstructured grids by spherical-harmonic (m=0) least squares.
 
@@ -54,6 +55,11 @@ class sph_zonal_averager:
         `dedup=True` (this build only) turns on the structure-exploiting fast path: columns sharing a latitude share a
         basis row (sph_zonal_mean.py:361-363), so fields are first reduced to per-latitude sums and every GEMM runs on
         the unique latitudes (721 instead of 1,038,240 columns on a 0.25-degree lat-lon grid).  Same results to rounding.
+        `min_norm=True` (this build only) accepts a rank-deficient basis, e.g. L+1 above the number of distinct
+        latitudes: the result is NumPy's minimum-norm least-squares solution, np.linalg.lstsq(Y0, ., rcond=None), whose
+        cutoff drops singular values <= eps * max(N, L+1) * sigma_1.  On a lat-lon grid the native mean is then the
+        per-latitude mean and the output mean the minimum-norm Legendre interpolant of those means.  `rank` is the
+        number of directions kept (L+1 on a full-rank grid).  Not available together with `weights`.
         '''
         self.L = L
         self.lat = lat.values if ar.is_dataarray(lat) else lat
@@ -83,13 +89,16 @@ class sph_zonal_averager:
         self.grid_name, self.grid_out_name = gname, goname
         self.Y0_file_out = None
         self.Y0p_file_out = None
+        if min_norm and weights is not None:
+            raise RuntimeError('min_norm=True is not available together with weights=')
         if not torch.cuda.is_available():
             raise RuntimeError('pytemdiags_b200 needs a CUDA device (sm_100a); there is no CPU fallback')
         if dedup and weights is not None:
             raise RuntimeError('dedup=True is not available together with weights=')
         self.dedup = bool(dedup)
+        self.min_norm = bool(min_norm)
         self._engine = _cached_engine(self.lat, self.lat_out, self.L, device, overwrite=overwrite, weights=self.weights,
-                                      dedup=self.dedup)
+                                      dedup=self.dedup, min_norm=self.min_norm)
         self._mats = None
 
     # ------------------------------------------------------------------
@@ -104,8 +113,14 @@ class sph_zonal_averager:
         self._mats = None
         if self.debug and self.weights is None:
             print('(sph_zonal_mean debug) Sanity check: sum(diag(Q^T Q)) = {} (should be {}); '
-                  'sum(offdiag) = {} (should be zero)'.format(self._engine.sanity[0], self.L + 1,
+                  'sum(offdiag) = {} (should be zero)'.format(self._engine.sanity[0], self._engine.rank,
                                                               self._engine.sanity[1]))
+
+    @property
+    def rank(self):
+        '''Number of basis directions the zonal mean uses: L+1, or the numerical rank of Y0 with min_norm=True
+        (None before sph_compute_matrices).'''
+        return self._engine.rank if self._engine.built else None
 
     def _export(self):
         if not self._engine.built:
