@@ -8,8 +8,7 @@
 // none of them reaches HBM.  Per CTA: BM (time,lev) rows, a split-K range of 16-column chunks.
 //
 //   per chunk:  GEMM1  E_f[BM x 16] = X_f - C_f[BM x lpad] * QT[lpad x 16]   f = u, v, theta, omega (theta: X = lev_scale * T;
-//                      the accumulators start from the X tile and the resident coefficients are negated),
-//               E_f written in place over the X tile
+//                      the accumulators start from the X tile and the resident coefficients are negated)
 //               GEMM2  acc_g[BM x lpad] += (E_a .* E_b)[BM x 16] * QT^T[16 x lpad]   g = uv, uw, v.theta
 //
 // Both GEMMs are DMMA.8x8x4; the QT chunk tile ([lpad rows][16 cols], TMA, 128-B swizzle) is the
@@ -17,11 +16,19 @@
 // C_f lives in shared memory for the CTA's lifetime (row-major, row stride = 4 or 12 mod 16
 // doubles so that the GEMM1 A fragments are bank-conflict-free under the mnmajor_k permutation).
 //
-// Warp organisation (measured choices, see DESIGN.md §6): 16 consumer warps + 1 TMA producer warp; the
-// 4 (BM=32) / 8 (BM=16) warps that own one 8-row m-tile form a group that synchronises on its own named
-// barrier for the GEMM1 -> GEMM2 hand-off; one barrier round covers two pipeline stages when four stages fit
-// (GEMM1 of both chunks shares the coefficient fragments).  BM = 32 / 16 / 8 rows for L+1 <= 104 / 208 / 408 is
-// dictated by the 4 x BM x lpad coefficient tile that must stay resident next to >= 2 pipeline stages.
+// Two consumer bodies (measured choices, see DESIGN.md §6); both have a TMA producer and a 2..6-stage mbarrier ring:
+//  * warp tiles (eddy_warp_tiles; the default TEM layout BM = 32 with 8 consumer warps, L+1 <= 104): each warp owns
+//    one 8-row m-tile and one 8-column half of every chunk and runs GEMM1 for all four fields, the products and GEMM2
+//    over its 8 columns from its own registers.  Nothing goes back to shared memory and warps never wait for each
+//    other inside the chunk loop; the two warps of an m-tile add their partial sums once, at the end.  A producer
+//    warpgroup lets setmaxnreg give the consumers the 240 registers the 3 x nt accumulator tiles need.
+//  * groups (every other layout: BM = 24 / 16 / 8, 16 consumer warps, the tracer pair, whose 4 x nt accumulator
+//    tiles do not fit in 240 registers): the 2..8 warps that own one 8-row m-tile each produce part of the
+//    eddies (GEMM1), write them in place over the X tile, meet at the group's named barrier and each run GEMM2 for
+//    a share of the degree tiles; one barrier round covers two pipeline stages when four stages fit (GEMM1 of both
+//    chunks shares the coefficient fragments).
+// BM = 32 / 16 / 8 rows for L+1 <= 104 / 208 / 408 is dictated by the 4 x BM x lpad coefficient tile that must stay
+// resident next to >= 2 pipeline stages.
 // Tried and rejected (slower): predicated per-(tile, product) work splitting to balance GEMM2 across a group
 // (27.0 vs 32.6 TFLOP/s: predicated DMMA + WARPSYNC), run-time selection between loop shapes inside one kernel
 // (ptxas schedules both worse; loop shapes are template parameters instead), splitting GEMM2 over k-steps as
@@ -98,18 +105,175 @@ __device__ __forceinline__ void eddy_gemm2(double (&acc)[NP][NJ][2], uint32_t st
     }
 }
 
+// The warp-tile body (eddy_warp_tiles below) serves the default TEM layout: BM = 32, 8 consumer warps, 3 products.
+template <int BM, int WARPS, int NP> constexpr bool eddy_warp_tile() { return BM == 32 && WARPS == 8 && NP == 3; }
+
 // Producer warps: with 16 consumer warps a single extra warp would put 5 warps on one SM sub-partition and cap every
 // thread at 96 registers (16384 / 5 / 32, rounded down to 8).  A full producer WARPGROUP instead lets the kernel
 // re-balance with setmaxnreg: the 4 producer warps drop to 24 registers, the 16 consumers rise to 112.  The CTA's
 // register pool is what it was launched with (640 threads x 96): 512 x 112 + 128 x 24 = 60416 <= 61440.  (A target
-// the pool cannot satisfy makes setmaxnreg.inc spin forever.)
-template <int WARPS> constexpr int eddy_producer_warps() { return WARPS == 16 ? 4 : 1; }
+// the pool cannot satisfy makes setmaxnreg.inc spin forever.)  The warp-tile body needs 156 registers of GEMM2
+// accumulators at nt = 13, more than the 224 of an 8 + 1 warp launch leave room for: it takes a producer warpgroup
+// too, 384 threads x 168 = 256 x 240 + 128 x 24.
+template <int BM, int WARPS, int NP> constexpr int eddy_producer_warps() {
+    return (WARPS == 16 || eddy_warp_tile<BM, WARPS, NP>()) ? 4 : 1;
+}
+
+// Per-CTA geometry shared by the producer and the consumer bodies.
+struct EddyCta {
+    uint32_t smem_base, bar_base, cs_base;
+    int stage_bytes, stages, row0, split, nloc;
+    __device__ __forceinline__ uint32_t full_bar(int s) const { return bar_base + 8u * s; }
+    __device__ __forceinline__ uint32_t empty_bar(int s) const { return bar_base + 8u * (ED_MAX_STAGES + s); }
+};
+
+// Bytes of shared memory the warp-tile body uses at the end of its split range to add the partial sums of the two
+// warps of each m-tile: 4 m-tiles x 3 products x nt tiles x 32 lanes x 16 B.  It reuses the drained stage ring, which
+// at BM = 32 holds >= 4 stages of 16 KB + 1 KB per degree tile (eddy_stages), i.e. always more than this.
+__host__ __device__ inline int eddy_exchange_bytes(int nt) { return 4 * 3 * nt * 32 * 16; }
+
+// Warp-tile consumer body for k_eddy<32, NJ, 8, TWO, 3> at a compile-time tile count NT = nt (<= 2 NJ).
+//   Consumer warp w owns m-tile mi = w / 2 (8 rows) and n8 half jn = w % 2 (8 columns) of every 16-column chunk, and
+//   takes that 8 x 8 tile from the X tile to the flux partial sums on its own:
+//   GEMM1     all four fields on the tile; the accumulators start from the X tile, Cs holds -C (as in the group body).
+//   products  u'v', u'omega', v'theta' from its own registers: the DMMA D fragment (lane (g, t) holds columns 2t, 2t+1
+//             of row g) is exactly the A fragment of two k4 steps of GEMM2 when the contraction visits {2t}, {2t + 1}.
+//   GEMM2     over its 8 columns into accumulators for all NT degree tiles of its 8 rows.
+// Nothing is written to a stage: no eddy tile, no group barrier, no proxy fence.  A warp releases a stage with a plain
+// mbarrier arrive after its last read, and the warps drift apart freely (one warp's GEMM1 runs under its neighbour's
+// GEMM2).  Bank conflicts: the X tile and GEMM1 use the group body's addressing (DMMA row g = physical row rho(g), the
+// mnmajor_k contraction order, natural columns).  The GEMM2 B fragment is one LDS.128 per degree tile (both columns
+// of a lane); with natural degree order the quarter-warp g = 2q, 2q + 1 would read QT rows 2q, 2q + 1, whose swizzled
+// 16-B chunks {jn*4 .. jn*4+3} ^ row coincide (2 ways).  DMMA column n therefore carries degree rho(n) of its n8
+// tile: the quarter-warp reads rows q and q + 4, whose chunks lie in opposite halves of the 128-B row (conflict-free,
+// like the X tile).  Accumulator element 0 / 1 of lane (g, t) is then degree t / t + 4 of row rho(g).
+template <int NT, bool TWO>
+__device__ __forceinline__ void eddy_warp_tiles(const EddyParams& p, const EddyCta& c, int warp, int lane) {
+    constexpr int BM = 32;
+    constexpr int XF_BYTES = BM * TILE_ROW_BYTES;
+    constexpr uint32_t Q_OFF = 4 * XF_BYTES;
+    const int g = lane >> 2, t = lane & 3;
+    const int mi = warp >> 1, jn = warp & 1;
+    const int rg = (g >> 1) | ((g & 1) << 2);   // rho(g)
+    double tscale = 1.0;
+    {
+        const int row = c.row0 + mi * 8 + rg;
+        if (p.lev_scale != nullptr && row < p.rows) tscale = p.lev_scale[row % p.nlev];
+    }
+    double acc[3][NT][2];
+#pragma unroll
+    for (int q = 0; q < 3; q++)
+#pragma unroll
+        for (int j = 0; j < NT; j++) acc[q][j][0] = acc[q][j][1] = 0.0;
+
+    const uint32_t x_off = swz_off(mi * 8 + rg, jn * 8 + 2 * t);
+    const uint32_t fstride = (uint32_t)(BM * p.ls) * 8u;                 // one field's Cs block
+    uint32_t a1_off[2], b1_off[2];                                       // GEMM1 fragments at k step cc of an l8 block
+#pragma unroll
+    for (int cc = 0; cc < 2; cc++) {
+        const int kin = mnmajor_k(t, cc);
+        a1_off[cc] = c.cs_base + (uint32_t)((mi * 8 + g) * p.ls + kin) * 8u;
+        b1_off[cc] = Q_OFF + (uint32_t)(kin * TILE_ROW_BYTES) + (uint32_t)((((jn * 4 + (g >> 1)) ^ kin) & 7) << 4) +
+                     (uint32_t)((g & 1) << 3);
+    }
+    const uint32_t b2_off = Q_OFF + (uint32_t)(rg * TILE_ROW_BYTES) + (uint32_t)((((jn * 4 + t) ^ rg) & 7) << 4);
+
+    auto round = [&](auto nch_tag, int i) {
+        constexpr int NCH = decltype(nch_tag)::value;
+        uint32_t st[NCH];
+#pragma unroll
+        for (int ch = 0; ch < NCH; ch++) {
+            const int s = (i + ch) % c.stages;
+            mbar_wait(c.full_bar(s), ((i + ch) / c.stages) & 1);
+            st[ch] = c.smem_base + s * c.stage_bytes;
+        }
+        // ---------------- GEMM1: E_f = X_f - C_f * QT, f = u, v, theta, omega, on this warp's 8 x 8 tile ----------------
+        double e[NCH][4][2];
+#pragma unroll
+        for (int ch = 0; ch < NCH; ch++)
+#pragma unroll
+            for (int f = 0; f < 4; f++) {
+                double2 x = lds128(st[ch] + f * XF_BYTES + x_off);
+                if (f == 2) { x.x *= tscale; x.y *= tscale; }
+                e[ch][f][0] = x.x;
+                e[ch][f][1] = x.y;
+            }
+#pragma unroll
+        for (int l8 = 0; l8 < NT; l8++) {
+#pragma unroll
+            for (int cc = 0; cc < 2; cc++) {
+                double a[4], b[NCH];
+#pragma unroll
+                for (int f = 0; f < 4; f++) a[f] = lds64(a1_off[cc] + f * fstride + (uint32_t)(l8 * 64));
+#pragma unroll
+                for (int ch = 0; ch < NCH; ch++) b[ch] = lds64(st[ch] + b1_off[cc] + (uint32_t)(l8 * 8 * TILE_ROW_BYTES));
+#pragma unroll
+                for (int ch = 0; ch < NCH; ch++)
+#pragma unroll
+                    for (int f = 0; f < 4; f++) dmma(e[ch][f][0], e[ch][f][1], a[f], b[ch]);
+            }
+        }
+        // ---------------- flux products and GEMM2: acc_g += P_g * QT^T over this warp's 8 columns ----------------
+#pragma unroll
+        for (int ch = 0; ch < NCH; ch++) {
+            double pr[2][3];   // [k4 step: column 2t / 2t + 1][u'v', u'omega', v'theta']
+#pragma unroll
+            for (int s = 0; s < 2; s++) {
+                pr[s][0] = e[ch][0][s] * e[ch][1][s];
+                pr[s][1] = e[ch][0][s] * e[ch][3][s];
+                pr[s][2] = e[ch][1][s] * e[ch][2][s];
+            }
+#pragma unroll
+            for (int j = 0; j < NT; j++) {
+                const double2 b = lds128(st[ch] + b2_off + (uint32_t)(j * 8 * TILE_ROW_BYTES));
+#pragma unroll
+                for (int q = 0; q < 3; q++) dmma(acc[q][j][0], acc[q][j][1], pr[0][q], b.x);
+#pragma unroll
+                for (int q = 0; q < 3; q++) dmma(acc[q][j][0], acc[q][j][1], pr[1][q], b.y);
+            }
+            __syncwarp();
+            if (lane == 0) mbar_arrive(c.empty_bar((i + ch) % c.stages));
+        }
+    };
+
+    int i = 0;
+    if constexpr (TWO) {
+        for (; i + 2 <= c.nloc; i += 2) round(std::integral_constant<int, 2>{}, i);
+    }
+    for (; i < c.nloc; i++) round(std::integral_constant<int, 1>{}, i);
+
+    // ---------------- split-K partials: the two warps of an m-tile add their sums through the drained ring ----------------
+    // Every consumer has passed the full barrier of every chunk of the range, so no TMA write is in flight.
+    named_bar_sync(15, 8 * 32);
+    const uint32_t xb = c.smem_base + (uint32_t)((mi * 3 * NT * 32 + lane) * 16);
+    if (jn == 1) {
+#pragma unroll
+        for (int q = 0; q < 3; q++)
+#pragma unroll
+            for (int j = 0; j < NT; j++) sts128(xb + (uint32_t)((q * NT + j) * 32 * 16), acc[q][j][0], acc[q][j][1]);
+    }
+    named_bar_sync(15, 8 * 32);
+    if (jn == 1) return;
+    const int row = c.row0 + mi * 8 + rg;
+    if (row < p.rows) {
+#pragma unroll
+        for (int q = 0; q < 3; q++) {
+            double* out = p.part + (((size_t)c.split * 3 + q) * p.rows + row) * (NT * 8);
+#pragma unroll
+            for (int j = 0; j < NT; j++) {
+                const double2 o = lds128(xb + (uint32_t)((q * NT + j) * 32 * 16));
+                out[j * 8 + t] = acc[q][j][0] + o.x;
+                out[j * 8 + t + 4] = acc[q][j][1] + o.y;
+            }
+        }
+    }
+}
 
 template <int BM, int NJ, int WARPS, bool TWO, int NP>
-__global__ void __launch_bounds__((WARPS + eddy_producer_warps<WARPS>()) * 32, 1)
+__global__ void __launch_bounds__((WARPS + eddy_producer_warps<BM, WARPS, NP>()) * 32, 1)
 k_eddy(const __grid_constant__ EddyMaps maps, const EddyParams p) {
     constexpr int MT = BM / 8;          // m8-tiles per CTA
-    constexpr int PW = eddy_producer_warps<WARPS>();
+    constexpr int PW = eddy_producer_warps<BM, WARPS, NP>();
     constexpr int NW2 = WARPS / MT;     // warps per m-tile group (2, 4, 8 or 16)
     // GEMM1: a group owns 8 units (4 fields x 2 n8-tiles of the 16-column chunk) of its m-tile
     //   NW2 = 2: 2 fields x 2 n-tiles per warp;  NW2 = 4: 2 fields x 1 n-tile (fewest LDS per DMMA once two chunks
@@ -168,7 +332,8 @@ k_eddy(const __grid_constant__ EddyMaps maps, const EddyParams p) {
     }
 
     // ------------------------------ consumers ------------------------------
-    if constexpr (PW == 4) asm volatile("setmaxnreg.inc.sync.aligned.u32 112;\n");
+    if constexpr (eddy_warp_tile<BM, WARPS, NP>()) asm volatile("setmaxnreg.inc.sync.aligned.u32 240;\n");
+    else if constexpr (PW == 4) asm volatile("setmaxnreg.inc.sync.aligned.u32 112;\n");
     const int g = lane >> 2, t = lane & 3;
     const int tid = threadIdx.x;   // 0 .. WARPS*32-1
     // spectral coefficients of the 4 fields for this CTA's rows -> Cs[f][r][LS]
@@ -188,6 +353,19 @@ k_eddy(const __grid_constant__ EddyMaps maps, const EddyParams p) {
     }
     (void)tid;
     named_bar_sync(15, WARPS * 32);
+
+    if constexpr (eddy_warp_tile<BM, WARPS, NP>()) {
+        const EddyCta c{smem_base, bar_base, cs_base, stage_bytes, STAGES, row0, split, nloc};
+        // NJ bounds the tile count (nt = 2 NJ - 1 or 2 NJ, and nt <= 13 at BM = 32): one loop shape per count
+        constexpr int NTM = 2 * NJ < 13 ? 2 * NJ : 13;
+        if constexpr (2 * NJ - 1 < NTM) {
+            if (p.nt == NTM) eddy_warp_tiles<NTM, TWO>(p, c, warp, lane);
+            else eddy_warp_tiles<NTM - 1, TWO>(p, c, warp, lane);
+        } else {
+            eddy_warp_tiles<NTM, TWO>(p, c, warp, lane);
+        }
+        return;
+    }
 
     // Warp roles.  The warps that produce the eddies of m-tile `mi` (GEMM1) are exactly the warps that
     // consume them (GEMM2), so the E hand-off needs only a barrier among that group, not the whole
@@ -386,7 +564,7 @@ static int launch_eddy_2(const EddyMaps& maps, const EddyParams& p, int smem, cu
     cudaError_t e = cudaFuncSetAttribute(k_eddy<BM, NJ, WARPS, TWO, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e != cudaSuccess) return (int)e;
     const int ntiles = (p.rows + BM - 1) / BM;
-    k_eddy<BM, NJ, WARPS, TWO, NP><<<ntiles * p.nsplit, (WARPS + eddy_producer_warps<WARPS>()) * 32, smem, stream>>>(maps, p);
+    k_eddy<BM, NJ, WARPS, TWO, NP><<<ntiles * p.nsplit, (WARPS + eddy_producer_warps<BM, WARPS, NP>()) * 32, smem, stream>>>(maps, p);
     return (int)cudaGetLastError();
 }
 
@@ -454,6 +632,8 @@ int launch_eddy_flux_project(const double* const* x4, int rows, int ncol, size_t
         if (rc) return temd_set_error(rc, "eddy_flux_project: tracer-pair kernel launch failed (nj %d)", nj);
         return launch_reduce_partials(part, coef_flux, nsplit, 4, rows, lpad, nullptr, -1, 1, stream);
     }
+    if (bm == 32 && warps == 8 && p.stages * (4 * bm + lpad) * TILE_ROW_BYTES < eddy_exchange_bytes(nt))
+        return temd_set_error(-1, "eddy_flux_project: stage ring too small for the partial-sum exchange (lpad = %d)", lpad);
     const int nw2 = warps / (bm / 8);
     const int nj = (nt + nw2 - 1) / nw2;
 #define ED_CASE(BM_, NJ_, W_) if (bm == BM_ && nj == NJ_ && warps == W_) rc = launch_eddy_t<BM_, NJ_, W_>(maps, p, smem, stream);
